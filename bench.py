@@ -2,7 +2,7 @@
 """bench.py -- VO frames/s of the DF-VO tracking hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference|torch_gpu]
-                    [--config vo|corr64|ransac10k|pairs64|parity] [--no-extras]
+                    [--config vo|corr64|ransac10k|pairs64|parity] [--no-extras] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Default workload (`--config vo`, BASELINE.json configs[1]): KITTI-odometry-shaped stream of 376x1241 RGB frames, full hybrid
@@ -69,7 +69,15 @@ def parse():
     ap.add_argument("--no-extras", action="store_true", help="skip precision modes / library baseline / extra configs / e2e_libs")
     ap.add_argument("--diag-no-track", action="store_true",
                     help="DIAGNOSTIC, not a bench value: replace the tracker by an identity pose to see the networks-only ceiling of the pipeline")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (the 4x4 float64 global pose) as DIR/pose.npy, "
+                         "so that two builds can be compared output for output on the same seeded inputs")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.config != "vo" or a.diag_no_track):
+        ap.error("--dump-outputs applies to the default workload (--impl b200 --config vo) only")
+    return a
 
 
 def dist_env():
@@ -702,6 +710,7 @@ def run_b200(args):
                 cs.wait_stream(sx)
         e1.record()
         barrier()
+        state["last_pose"] = pose
         if clocks:
             clocks.mark(False)
         ms = e0.elapsed_time(e1)
@@ -728,6 +737,10 @@ def run_b200(args):
         clocks.start()
     ms, launches, _ = timed(pipe, args.steps, True, clocks if rank == 0 else None)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the warm-up is longer than the pipeline's lag, so every timed step returns a pose
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "pose.npy"), np.asarray(state["last_pose"], np.float64))
     ms_e2e, _, lat_e2e = timed(pipe, args.steps, False)
     h2d, d2h = state["h2d"] / args.steps, state["d2h"] / args.steps
     pipe.flush()
